@@ -8,10 +8,14 @@ One "step" = one full pass of the hot path over one batch: 250 denoising steps f
 Independent prompts shard across GPUs with no data-path collective (weak scaling); the finished
 latents are all-gathered once per step (tiny).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
-`--impl reference` times the reference algorithm's CPU path (the oracle port -- /root/reference
-is a Python tree that cannot travel to the GPU box) on a bounded sample of the same workload.
+`--impl reference` times the reference algorithm's CPU path (the oracle port of the reference's
+Python modules) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step returned, the denoised latents of the batch
+(all ranks' latents after the gather), as DIR/latents.npy in float32.  The inputs are drawn from
+fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -44,7 +48,14 @@ def parse():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--denoise-steps", type=int, default=DENOISE_STEPS, help=argparse.SUPPRESS)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the latents of the last timed step to DIR/latents.npy (float32)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs is only available with --impl ours")
+    return a
 
 
 def workload_config(n_gpus):
@@ -274,12 +285,14 @@ def run_ours(args):
     model.prepare()
     tables = pipeline.edm_cfg_tables(nsteps, CFG_SCALE, B, dev)
     gathered = torch.empty(n_gpus * B, 12, 32, 32, device=dev) if world > 1 else None
+    last = {}
 
     def one_step_device():
         lat = pipeline.sample_t23d(model, randn_d, {"crossattn": ctx_d}, {"crossattn": uc_d}, nsteps,
                                    CFG_SCALE, tables)
         if world > 1:
             dist.all_gather_into_tensor(gathered, lat)
+        last["latents"] = gathered if world > 1 else lat
         return lat
 
     def one_step_e2e():
@@ -319,6 +332,10 @@ def run_ours(args):
         clocks.start()
     ms_total, launches = timed(one_step_device, args.steps, args.warmup)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "latents.npy"), last["latents"].float().cpu().numpy())
     ms_step = ms_total / args.steps
     value = B * n_gpus / (ms_step / 1e3)
 

@@ -188,24 +188,71 @@ def test_identical_token_row_detection(monkeypatch):
     assert _attention_rows(torch.cat([same, c])) is None
 
 
-def test_overlay_lets_the_reference_script_utils_import():
-    """With the hook installed, the reference's OWN `guided_diffusion/script_util.py` and `nsr/script_util.py`
-    import: mirrored names resolve to this package, the names the mirrors do not define
-    (ViTTriplaneDecomposed, Encoder, MVEncoder, ImageCondDiTBlock, Triplane_fg_bg_plane, ...) fall back to the
-    reference's files.  Needs the reference checkout (build container only) and the third-party stubs."""
+_SCRIPT_UTIL_CHECKOUT = {
+    # a stand-in checkout laid out like the reference's: its script_util modules import mirrored and
+    # non-mirrored names side by side, as the reference's guided_diffusion/ and nsr/script_util.py do
+    "dit/dit_models_xformers.py": "class TextCondDiTBlock:\n    pass\n\n\nclass ImageCondDiTBlock:\n    pass\n",
+    "dit/dit_trilatent.py": "DiT_models = {}\n",
+    "dit/dit_i23d.py": "DiT_models = {}\n",
+    "nsr/triplane.py": "class Triplane:\n    pass\n\n\nclass Triplane_fg_bg_plane(Triplane):\n    pass\n",
+    "vit/vit_triplane.py": "from nsr.triplane import Triplane  # noqa: F401  (re-export)\n\n\n"
+                           "class ViTTriplaneDecomposed:\n    pass\n",
+    "ldm/modules/diffusionmodules/model.py": "class Encoder:\n    pass\n\n\nclass MVEncoder(Encoder):\n    pass\n",
+    "nsr/script_util.py": "from vit.vit_triplane import Triplane, ViTTriplaneDecomposed  # noqa: F401\n"
+                          "from nsr.triplane import Triplane_fg_bg_plane  # noqa: F401\n"
+                          "from ldm.modules.diffusionmodules.model import Encoder, MVEncoder  # noqa: F401\n",
+    "guided_diffusion/script_util.py": '''\
+from . import gaussian_diffusion as gd
+from .respace import SpacedDiffusion, space_timesteps
+from dit.dit_models_xformers import TextCondDiTBlock, ImageCondDiTBlock  # noqa: F401
+from dit.dit_trilatent import DiT_models as DiT_models_t23d
+from dit.dit_i23d import DiT_models as DiT_models_i23d
+
+
+def model_and_diffusion_defaults():
+    return dict(create_dit=False, i23d=False, dit_model_arch="DiT-L/2", context_dim=768, roll_out=False,
+                denoise_in_channels=4, denoise_out_channels=4, diffusion_input_size=32, learn_sigma=False,
+                mixed_prediction=False, diffusion_steps=1000, timestep_respacing="")
+
+
+def create_model_and_diffusion(create_dit, i23d, dit_model_arch, context_dim, roll_out, denoise_in_channels,
+                               diffusion_input_size, learn_sigma, diffusion_steps, timestep_respacing, **kw):
+    assert create_dit
+    common = dict(input_size=diffusion_input_size, num_classes=0, learn_sigma=learn_sigma,
+                  in_channels=denoise_in_channels, context_dim=context_dim, roll_out=roll_out)
+    if i23d:
+        model = DiT_models_i23d[dit_model_arch](pooling_ctx_dim=768, **common)
+    else:
+        model = DiT_models_t23d[dit_model_arch](vit_blk=TextCondDiTBlock, **common)
+    diffusion = SpacedDiffusion(use_timesteps=space_timesteps(diffusion_steps, timestep_respacing or str(diffusion_steps)),
+                                betas=gd.get_named_beta_schedule("linear", diffusion_steps),
+                                model_mean_type=gd.ModelMeanType.EPSILON, model_var_type=gd.ModelVarType.FIXED_LARGE,
+                                loss_type=gd.LossType.MSE)
+    return model, diffusion
+''',
+}
+
+
+def test_overlay_lets_the_reference_script_utils_import(tmp_path):
+    """With the hook installed, a checkout's `guided_diffusion/script_util.py` and `nsr/script_util.py` laid out
+    like the reference's import: mirrored names resolve to this package, the names the mirrors do not define
+    (ViTTriplaneDecomposed, Encoder, MVEncoder, ImageCondDiTBlock, Triplane_fg_bg_plane) fall back to the
+    checkout's files, and the checkout's own factory builds the mirrors."""
     import importlib
-    import os
     import sys
     import pytest
-    if not os.path.isdir("/root/reference/nsr"):
-        pytest.skip("reference checkout not present (GPU box)")
-    prefixes = ("dit", "sgm", "nsr", "guided_diffusion", "transport", "vit", "ldm", "xformers", "timm", "torchdiffeq",
-                "omegaconf", "blobfile")
+    for rel, text in _SCRIPT_UTIL_CHECKOUT.items():
+        d = tmp_path
+        for part in rel.split("/")[:-1]:
+            d = d / part
+            d.mkdir(exist_ok=True)
+            (d / "__init__.py").touch()
+        (tmp_path / rel).write_text(text)
+    prefixes = ("dit", "sgm", "nsr", "guided_diffusion", "transport", "vit", "ldm")
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k.split(".")[0] in prefixes}
     saved_path = list(sys.path)
-    from oracle import _stubs
     from ln3diff_b200 import overlay
-    _stubs.install()
+    sys.path.insert(0, str(tmp_path))
     overlay.install()
     try:
         g = importlib.import_module("guided_diffusion.script_util")
@@ -221,7 +268,7 @@ def test_overlay_lets_the_reference_script_utils_import():
         assert n.Triplane_fg_bg_plane.__module__ == "nsr.triplane"
         with pytest.raises(AttributeError):
             importlib.import_module("dit.dit_trilatent").no_such_name
-        # the reference's own factory, unmodified, now builds the mirrors (guided_diffusion/script_util.py:152-252)
+        # the checkout's own factory, unmodified, now builds the mirrors
         d = g.model_and_diffusion_defaults()
         d.update(dict(create_dit=True, dit_model_arch="DiT-B/2", context_dim=768, roll_out=True, denoise_in_channels=4,
                       denoise_out_channels=4, diffusion_input_size=32, learn_sigma=False, mixed_prediction=False,
