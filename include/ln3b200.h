@@ -107,10 +107,10 @@ typedef struct ln3_fmha_args {
   int B, H, Lq, Lkv, head_dim;
   long long q_ld, q_bs, k_ld, k_bs, v_ld, v_bs, o_ld, o_bs; /* elements */
   float scale;
-  /* optional second K/V source appended after the first along the sequence (Lkv must then be a
-   * multiple of 128 for the two-warpgroup kernel; the default kernel takes any Lkv): the step-invariant DINO tokens the I23D blocks concatenate to the latent
-   * tokens for self-attention (dit/dit_models_xformers.py:522-530) -- their K/V are cached per
-   * prompt and never copied.  k2/v2 NULL -> unused. */
+  /* optional second K/V source appended after the first along the sequence: the step-invariant DINO
+   * tokens the I23D blocks concatenate to the latent tokens for self-attention
+   * (dit/dit_models_xformers.py:522-530) -- their K/V are cached per prompt and never copied.
+   * k2/v2 NULL -> unused. */
   const void* k2;
   const void* v2;
   int Lkv2;

@@ -1,110 +1,85 @@
-// Fused multi-head attention forward for sm_100a (head_dim 64, bf16 in, fp32 softmax/accumulate).
+// Fused multi-head attention forward for sm_100a (head_dim 64, bf16 in, fp32 softmax / accumulate).
 //
-// Replaces xformers.ops.memory_efficient_attention at its three call sites on the path:
+// Replaces xformers.ops.memory_efficient_attention at its call sites on the path:
 //   vit/vision_transformer.py:114-118 (DiT self-attention, (B, N, 3, H, 64) packed qkv),
 //   ldm/modules/attention.py:279-307  (cross-attention; the reference's three permute+contiguous
 //                                       copies disappear: heads are addressed through the TMA map),
 //   dit/dit_decoder.py                (in-plane / global attention of the DiT2 VAE decoder).
-// Semantics: out = softmax(q k^T * scale) v, no mask (xformers FMHA with attn_bias=None).
+// Semantics: out = softmax(q k^T * scale) v (xformers FMHA with attn_bias=None); optionally a causal mask
+// (CLIP text tower) or a second K/V source appended after the first (I23D DINO tokens, never concatenated).
 //
-// Warp-specialised, one CTA = 256 query rows (two 128-row tiles) of one (batch, head):
-//   warps 0-3 / 4-7 : softmax warpgroup of tile 0 / 1; thread r owns query row r (= TMEM lane r), so
-//                     the row max / sum need no cross-thread reduction.  S (128 fp32) is read once
-//                     from TMEM into registers, P = exp2(S*scale - m) goes to 128B-swizzled smem as bf16.
-//   warp 8          : TMA producer (Q double buffered per item, K/V ring of 3 blocks)
-//   warp 9          : tcgen05.mma issuer:  S_t = Q_t K^T (128x128x16 x4),  O_t += P_t V (128x64x16 x8,
-//                     V MN-major straight from the TMA layout).  S_t of block g+1 is issued as soon as
-//                     the warpgroup has pulled S_t of block g into registers (s_empty), i.e. BEFORE its
-//                     exponentials, so a warpgroup never waits for the tensor core in steady state.
-// The softmax is MUFU-bound at head_dim 64 (16 ex2/clk/SM against 2 x 128x128 elements per step), so
-// kPolyPer8 of every 8 exponentials are evaluated on the FMA pipe instead (Cody-Waite split + degree-3
-// minimax polynomial, rel. error 8.8e-5 -- below the bf16 rounding of P).
-// O accumulates in TMEM across KV blocks.  The running max is only refreshed when it grew by more
-// than 2^8 (then the owning thread rescales its O row in TMEM); otherwise P is computed against the
-// stale max, which is exact after the final 1/l normalisation.
+// Why three softmax warpgroups.  At head_dim 64 the softmax is bound by the XU (MUFU.EX2: 16 lanes/clk/SM, i.e.
+// one warp instruction per 8 clocks per scheduler) at twice the tensor time.  An in-kernel timeline of a CTA with two
+// softmax warpgroups (profiles/r2_fmha_timeline_self.txt) shows the XU pipe saturated only while BOTH warpgroups are
+// inside their exponential loops and idle for about a third of every block period (TMEM load, row maximum, barrier
+// round trips), because the two fall into lock-step; a single warp per scheduler cannot keep the pipe busy on its own
+// (ptxas batches the MUFUs, an in-order warp then has nothing else to issue).  Here a CTA owns THREE 128-row query
+// tiles (one warpgroup each, 12 softmax warps = 3 per scheduler), so while one warpgroup does its bookkeeping the
+// other two can keep the XU busy.  KV blocks are 96 rows so that 3 score tiles (3 x 96 fp32 columns) and 3 output
+// tiles (3 x 64) fit the 512 TMEM columns; a thread holds 96 scores.  ptxas (CUDA 12.9) reports 128 registers, a
+// 72-byte stack frame, 32 bytes of spill stores and 52 bytes of spill loads.
+//
+// Roles (512 threads): warps 0-11 softmax (warpgroup t = warp / 4 owns query tile t, thread = row = TMEM
+// lane), warp 12 TMA producer, warps 13-15 tcgen05.mma issuers (one per tile).
+//   TMA : Q (3 tiles, single buffer per item), K ring and V ring (3 stages each, released separately: K of a
+//         block is dead two block periods before its V).
+//   MMA : S_t(g) = Q_t K(g)^T (128x96x16 x4), O_t += P_t(g) V(g) (128x64x16 x6, V MN-major from the TMA
+//         layout).  Issue order per tile: P_t V(g), then Q_t K(g+2)^T as soon as the warpgroup has pulled
+//         S_t(g+1) into registers.
+// O accumulates in TMEM across KV blocks.  The running maximum is only raised when a block exceeds it by more than
+// 2^8 (then the owning thread rescales its O row in TMEM); otherwise P is computed against the stale maximum, which
+// is exact after the final 1/l normalisation.  Only the first block of an item pays a separate max pass; later
+// blocks track their maximum inside the exponential loop and are redone in the rare case that it passes the
+// threshold.
+// Work items are (batch, head, 384-query-row) triples dealt round-robin to a persistent grid; the last,
+// partial round is dealt as (2 tiles | 1 tile) halves to twice as many SMs when they fit.
 #include <type_traits>
-
-#include <cstdlib>
 
 #include "common.cuh"
 #include "ln3_internal.h"
 
 namespace ln3 {
 
-int fmha3_launch(const ln3_fmha_args* a, int variant, cudaStream_t stream);  // attention3_tcgen05.cu
-
-static constexpr int kQT = 128;   // query rows per tile (2 tiles per CTA)
-static constexpr int kKT = 128;   // kv rows per block
-static constexpr int kHD = 64;    // head dim
-static constexpr int kTileBytes = 128 * kHD * 2;  // 16 KB
-static constexpr int kKVStages = 3;
-// Q[2 buffers][2 tiles] | K[3] | V[3] | P0 (2 atoms) P1 (2 atoms)
-static constexpr int kFmhaSmem = 1024 + kTileBytes * (4 + 2 * kKVStages + 4) + 256;
-static constexpr int kPolyPer8Default = 0;  // exponentials per 8 evaluated on the FMA pipe (LN3_FMHA_POLY)
+static constexpr int kQT = 128;    // query rows per tile
+static constexpr int kNT = 3;      // query tiles (= softmax warpgroups) per CTA
+static constexpr int kKB = 96;     // kv rows per block
+static constexpr int kHD = 64;     // head dim
+static constexpr int kQBytes = kQT * kHD * 2;    // 16 KB
+static constexpr int kKVBytes = kKB * kHD * 2;   // 12 KB
+static constexpr int kStages = 3;                // K ring and V ring depth
+static constexpr int kPBytes = 2 * kQBytes;      // P_t: two 64-column 128B-swizzle atoms (the second half used)
+static constexpr int kSmem = 1024 + kNT * kQBytes + 2 * kStages * kKVBytes + kNT * kPBytes + 512;
+static constexpr int kThreads = (4 * kNT + 1 + kNT) * 32;  // 512: 12 softmax warps, TMA warp, 3 MMA warps
+static constexpr int kTmemCols = 512;            // S_t at 96 t (t < 3), O_t at 288 + 64 t
+static constexpr int kTmemO = kNT * kKB;
+static constexpr float kRescaleThreshold = 8.0f;  // log2 units
+// Suspend-time hint of every mbarrier wait: a waiting warp sleeps in hardware instead of feeding try_wait / branch
+// pairs into the issue slots of the softmax warps it shares a scheduler with (measured against plain polling:
+// DESIGN.md section 5c).
+static constexpr uint32_t kWaitNs = 2000;
 
 #ifdef LN3_FMHA_TRACE
-// Debug timeline (tools/microbench/fmha_trace.cu): CTA 0, first 64 KV blocks; role 0/1 = softmax
-// warpgroup 0/1 (thread 0 of the group), role 2 = MMA thread; 8 clock64 slots per block.
-__device__ long long g_fmha_trace[3][64][12];
-#define LN3_TR(role, blk, slot)                                                          \
-  do {                                                                                   \
-    if (blockIdx.x == 0 && (blk) < 64) g_fmha_trace[role][blk][slot] = clock64();        \
+// Debug timeline (tools/microbench/fmha_trace.cu): CTA 0, first 64 KV blocks; role 0-2 = softmax warpgroups
+// (thread 0 of the group), role 3 = MMA.
+__device__ long long g_fmha_trace[4][64][12];
+#define LN3_TR3(role, blk, slot)                                                   \
+  do {                                                                             \
+    if (blockIdx.x == 0 && (blk) < 64) g_fmha_trace[role][blk][slot] = clock64();  \
   } while (0)
 #else
-#define LN3_TR(role, blk, slot) do {} while (0)
+#define LN3_TR3(role, blk, slot) do {} while (0)
 #endif
 
-// 2^x for x <= ~8 on the FMA pipe: x = floor(x) + f, 2^f by a degree-3 minimax polynomial, the integer
-// part added straight into the exponent field (the round-down add leaves floor(x) in the low mantissa
-// bits of t).  x is clamped at -126 (result 2^-126 instead of 0: irrelevant after the bf16 rounding).
-__device__ __forceinline__ float exp2_poly(float x) {
-  x = fmaxf(x, -126.f);
-  float t;
-  asm("add.rm.ftz.f32 %0, %1, %2;" : "=f"(t) : "f"(x), "f"(12582912.f));
-  const float f = x - (t - 12582912.f);
-  float q = fmaf(f, 0.077119089663028717041015625f, 0.227564394474029541015625f);
-  q = fmaf(f, q, 0.695146143436431884765625f);
-  q = fmaf(f, q, 1.f);
-  return __uint_as_float(__float_as_uint(q) + (__float_as_uint(t) << 23));
-}
-static constexpr int kFmhaTmemCols = 512;  // S0 [0,128) S1 [128,256) O0 [256,320) O1 [320,384)
-static constexpr int kFmhaThreads = 320;
-static constexpr float kRescaleThreshold = 8.0f;  // log2 units
-
 struct FmhaParams {
-  int Lq, Lkv;
-  int Lkv2;  // rows of the optional second K/V source (0 = none)
-  int B, H, nq;  // work items = B * H * nq query-row pairs (256 rows each)
-  float rcp_nq, rcp_H;  // 1 / nq, 1 / H (item index decomposition)
-  float scale_log2;  // softmax scale * log2(e)
-  // Tail schedule (MMA2 kernels): items [0, full_items) are dealt round-robin as 256-row pairs; the
-  // n_split = nitems - full_items items of the last, partial round are dealt as single 128-row tiles to CTAs
-  // 0 .. 2*n_split-1 (CTA c: item full_items + c/2, tile c & 1).  n_split = 0: plain round-robin.
-  int full_items, n_split;
+  int Lq, Lkv, Lkv2;
+  int B, H, nq;          // work items = B * H * nq query-row triples (384 rows each)
+  float rcp_nq, rcp_H;
+  float scale_log2;
+  int full_items, n_split;  // tail schedule: see the file header
+  int causal;               // key j visible to query i only when j <= i
 };
 
-// Persistent: each CTA walks work items w = blockIdx.x, +gridDim.x, ... (item = one (batch, head,
-// 256-query-row pair)); barriers, TMEM and the K/V ring carry over between items and Q is double
-// buffered, so the TMA warp prefetches the next item's Q / K / V while the current item is still in its
-// softmax -- the per-CTA prologue (TMEM allocation, barrier init, first-load latency) is paid once per
-// SM instead of once per item (it was ~30 % of a self-attention item and most of a cross-attention one).
-// SPLIT = true: 16 softmax warps instead of 8 -- every 128-row tile is handled by TWO warpgroups, each
-// owning 64 of the 128 score columns of a block (= one 64-column P atom).  Four softmax warps per scheduler
-// instead of two cover each other's MUFU / barrier / TMEM latencies, and a thread holds 64 scores instead
-// of 128 (no spills, room to interleave).  The two halves of a row agree on the block maximum and the final
-// row sum through spare TMEM columns [384, 400) (lane = row, so partner warps address the same lanes).
-// MMA2 = true: one tcgen05.mma issue warp PER query tile instead of one for both.  A single in-order issue
-// warp couples the two softmax warpgroups (QK_1(g+1) waits for warpgroup 1 to have read S_1(g) before P_0 V(g)
-// can be issued, so a lagging warpgroup stalls its sibling's o_full); with two issue warps each tile's
-// S -> P -> O chain only depends on its own warpgroup.  MMA2 kernels also use the tail schedule of FmhaParams.
-template <bool SPLIT, bool MMA2 = false>
-constexpr int fmha_threads() { return SPLIT ? 576 : (MMA2 ? kFmhaThreads + 32 : kFmhaThreads); }
-
-// PTMEM = true: P_t is written to tensor memory (columns 384 + 64 t, bf16 pairs per 32-bit column) and fed
-// to P_t V as the TMEM A operand: no st.shared / proxy fence for P, and the N = 64 MMA no longer re-reads a
-// 4 KB A slice from shared memory per k-step.
-template <int kPolyPer8, bool PINGPONG, bool SPLIT = false, bool PTMEM = false, bool MMA2 = false>
-__global__ void __launch_bounds__(fmha_threads<SPLIT, MMA2>(), 1)
+__global__ void __launch_bounds__(kThreads, 1)
 fmha_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                 const __grid_constant__ CUtensorMap tmap_v, const __grid_constant__ CUtensorMap tmap_k2,
                 const __grid_constant__ CUtensorMap tmap_v2, const __grid_constant__ CUtensorMap tmap_o,
@@ -112,46 +87,51 @@ fmha_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) &
                                              ~static_cast<uintptr_t>(1023));
-  uint8_t* sQ = smem;                  // [2 buffers][2 tiles]
-  uint8_t* sK = sQ + 4 * kTileBytes;           // [kKVStages]
-  uint8_t* sV = sK + kKVStages * kTileBytes;   // [kKVStages]
-  uint8_t* sP = sV + kKVStages * kTileBytes;   // [2 tiles][2 atoms]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sP + 4 * kTileBytes);
-  uint64_t* q_full = bars;         // [2]
-  uint64_t* q_empty = bars + 2;    // [2]
-  uint64_t* kv_full = bars + 4;    // [kKVStages]
-  uint64_t* kv_empty = bars + 8;   // [kKVStages]
-  uint64_t* s_full = bars + 12;    // [2 tiles]
-  uint64_t* s_empty = bars + 14;   // [2 tiles], 128 arrivals: S_t is in registers
-  uint64_t* p_full = bars + 16;    // [2 tiles], 128 arrivals
-  uint64_t* o_full = bars + 18;    // [2 tiles]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 20);
+  uint8_t* sQ = smem;                          // [kNT]
+  uint8_t* sK = sQ + kNT * kQBytes;            // [kStages]
+  uint8_t* sV = sK + kStages * kKVBytes;       // [kStages]
+  uint8_t* sP = sV + kStages * kKVBytes;       // [kNT][2 atoms]
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sP + kNT * kPBytes);
+  uint64_t* q_full = bars;                     // [1]
+  uint64_t* q_empty = bars + 1;                // [1]
+  uint64_t* k_full = bars + 2;                 // [kStages]
+  uint64_t* k_empty = k_full + kStages;
+  uint64_t* v_full = k_empty + kStages;
+  uint64_t* v_empty = v_full + kStages;
+  uint64_t* s_full = v_empty + kStages;        // [kNT]
+  uint64_t* s_empty = s_full + kNT;            // [kNT] 4 arrivals (one per warp): S_t is in registers
+  uint64_t* p_full = s_empty + kNT;            // [kNT] 4 arrivals
+  uint64_t* o_full = p_full + kNT;             // [kNT]
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(o_full + kNT);
 
   const int tid = threadIdx.x;
   const int warp = tid >> 5;
-  constexpr int kSoftWarps = SPLIT ? 16 : 8;
-  constexpr int kTmaWarp = kSoftWarps, kMmaWarp = kSoftWarps + 1;
-  constexpr int kTileThreads = SPLIT ? 256 : 128;  // softmax threads per query tile
-  const int nkv1 = (p.Lkv + kKT - 1) / kKT;  // with a second source Lkv is a multiple of 128
-  const int nkv = nkv1 + (p.Lkv2 + kKT - 1) / kKT;
-  const int nitems = p.B * p.H * p.nq;
-  // w = (batch * H + head) * nq + qp; divisions by reciprocal multiply (exact for w < 2^20, checked on
-  // the host): a 32-bit integer division is ~150 dependent cycles and sat on every item boundary.
+  constexpr int kTmaWarp = 4 * kNT, kMmaWarp = 4 * kNT + 1;
+  const int nkv1 = (p.Lkv + kKB - 1) / kKB;  // a ragged last block of the first source is masked like the final one
+  const int nkv = nkv1 + (p.Lkv2 + kKB - 1) / kKB;
+  // w = (batch * H + head) * nq + qp; reciprocal multiplies (exact for w < 2^20, checked on the host)
   auto item_coords = [&](int w, int& q0, int& head, int& batch) {
     const int bh = __float2int_rz((static_cast<float>(w) + 0.5f) * p.rcp_nq);
     const int qp = w - bh * p.nq;
-    q0 = qp * 2 * kQT;
+    q0 = qp * kNT * kQT;
     batch = __float2int_rz((static_cast<float>(bh) + 0.5f) * p.rcp_H);
     head = bh - batch * p.H;
   };
-  // this CTA's schedule: n_full_my round-robin pair items, then (tail schedule) at most one single-tile item
+  // this CTA's schedule: n_full_my round-robin triple items, then (tail schedule) at most one partial item
   const int cta = static_cast<int>(blockIdx.x), ncta = static_cast<int>(gridDim.x);
   const int n_full_my = cta < p.full_items ? (p.full_items - cta + ncta - 1) / ncta : 0;
-  const bool has_half = cta < 2 * p.n_split;
-  const int n_my = n_full_my + (has_half ? 1 : 0);
-  auto sched = [&](int it, int& w, int& mask) {
-    if (it < n_full_my) { w = cta + it * ncta; mask = 3; }
-    else { w = p.full_items + (cta >> 1); mask = 1 << (cta & 1); }
+  const int n_my = n_full_my + (cta < 2 * p.n_split ? 1 : 0);
+  // item `it` of this CTA: work item, its coordinates and the set of tiles this CTA computes (0 = nothing)
+  auto sched = [&](int it, int& q0, int& head, int& batch) -> int {
+    int w, mask;
+    if (it < n_full_my) { w = cta + it * ncta; mask = 7; }
+    else { w = p.full_items + (cta >> 1); mask = (cta & 1) ? 4 : 3; }
+    item_coords(w, q0, head, batch);
+    int valid = 0;
+#pragma unroll
+    for (int t = 0; t < kNT; ++t)
+      if (q0 + t * kQT < p.Lq) valid |= 1 << t;
+    return mask & valid;
   };
 
   if (tid == 0) {
@@ -163,22 +143,24 @@ fmha_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       tma_prefetch_desc(&tmap_k2);
       tma_prefetch_desc(&tmap_v2);
     }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&q_full[i], 1);
-      mbar_init(&q_empty[i], MMA2 ? 2 : 1);
-      mbar_init(&s_full[i], 1);
-      mbar_init(&s_empty[i], kTileThreads);
-      mbar_init(&p_full[i], kTileThreads);
-      mbar_init(&o_full[i], 1);
+    mbar_init(q_full, 1);
+    mbar_init(q_empty, kNT);          // one release per MMA warp
+    for (int i = 0; i < kStages; ++i) {
+      mbar_init(&k_full[i], 1);
+      mbar_init(&k_empty[i], kNT);
+      mbar_init(&v_full[i], 1);
+      mbar_init(&v_empty[i], kNT);
     }
-    for (int i = 0; i < kKVStages; ++i) {
-      mbar_init(&kv_full[i], 1);
-      mbar_init(&kv_empty[i], MMA2 ? 2 : 1);
+    for (int i = 0; i < kNT; ++i) {
+      mbar_init(&s_full[i], 1);
+      mbar_init(&s_empty[i], 4);   // one arrival per softmax warp (elected lane after __syncwarp)
+      mbar_init(&p_full[i], 4);
+      mbar_init(&o_full[i], 1);
     }
     fence_barrier_init();
   }
   if (warp == kMmaWarp) {
-    tmem_alloc(tmem_slot, kFmhaTmemCols);
+    tmem_alloc(tmem_slot, kTmemCols);
     tmem_relinquish();
   }
   tc_fence_before();
@@ -191,260 +173,251 @@ fmha_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
   if (warp == kTmaWarp) {
     // ------------------------------------------------------------ TMA producer
     if ((tid & 31) == 0) {
-      int kst = 0, kph = 0;
+      int st = 0, ph = 0, n_items = 0;
       for (int it = 0; it < n_my; ++it) {
-        int w, mask, q0, head, batch;
-        sched(it, w, mask);
-        item_coords(w, q0, head, batch);
-        const int qb = it & 1;
-        mbar_wait(&q_empty[qb], ((it >> 1) & 1) ^ 1);
-        mbar_arrive_expect_tx(&q_full[qb], (mask == 3 ? 2 : 1) * kTileBytes);
-        for (int t = 0; t < 2; ++t)
-          if (mask >> t & 1)
-            tma_load_3d(sQ + (qb * 2 + t) * kTileBytes, &tmap_q, &q_full[qb], head * kHD, q0 + t * kQT, batch);
+        int q0, head, batch;
+        const int mask = sched(it, q0, head, batch);
+        if (mask == 0) continue;
+        mbar_wait_hint(q_empty, (n_items & 1) ^ 1, kWaitNs);
+        ++n_items;
+        mbar_arrive_expect_tx(q_full, __popc(mask) * kQBytes);
+        for (int t = 0; t < kNT; ++t)
+          if (mask >> t & 1) tma_load_3d(sQ + t * kQBytes, &tmap_q, q_full, head * kHD, q0 + t * kQT, batch);
         for (int j = 0; j < nkv; ++j) {
-          const int b = kst;
-          mbar_wait(&kv_empty[b], kph ^ 1);
-          if (++kst == kKVStages) kst = 0, kph ^= 1;
-          mbar_arrive_expect_tx(&kv_full[b], 2 * kTileBytes);
-          if (j < nkv1) {
-            tma_load_3d(sK + b * kTileBytes, &tmap_k, &kv_full[b], head * kHD, j * kKT, batch);
-            tma_load_3d(sV + b * kTileBytes, &tmap_v, &kv_full[b], head * kHD, j * kKT, batch);
-          } else {
-            tma_load_3d(sK + b * kTileBytes, &tmap_k2, &kv_full[b], head * kHD, (j - nkv1) * kKT, batch);
-            tma_load_3d(sV + b * kTileBytes, &tmap_v2, &kv_full[b], head * kHD, (j - nkv1) * kKT, batch);
-          }
+          const CUtensorMap* mk = j < nkv1 ? &tmap_k : &tmap_k2;
+          const CUtensorMap* mv = j < nkv1 ? &tmap_v : &tmap_v2;
+          const int r0 = (j < nkv1 ? j : j - nkv1) * kKB;
+          mbar_wait_hint(&k_empty[st], ph ^ 1, kWaitNs);
+          mbar_arrive_expect_tx(&k_full[st], kKVBytes);
+          tma_load_3d(sK + st * kKVBytes, mk, &k_full[st], head * kHD, r0, batch);
+          mbar_wait_hint(&v_empty[st], ph ^ 1, kWaitNs);
+          mbar_arrive_expect_tx(&v_full[st], kKVBytes);
+          tma_load_3d(sV + st * kKVBytes, mv, &v_full[st], head * kHD, r0, batch);
+          if (++st == kStages) st = 0, ph ^= 1;
         }
       }
     }
-  } else if (warp == kMmaWarp || (MMA2 && warp == kMmaWarp + 1)) {
-    // ------------------------------------------------------------ MMA issuer(s)
-    // The whole warp walks this loop with warp-uniform values (so descriptors live in uniform
-    // registers); elect_one_sync() guards only the tcgen05 instructions themselves.
-    // MMA2: this warp issues for query tile t_lo only; the sibling warp takes the other tile.
-    const int t_lo = MMA2 ? warp - kMmaWarp : 0;
-    const int t_hi = MMA2 ? t_lo + 1 : 2;
-    {
-      constexpr uint32_t idesc_s = make_idesc_bf16(128, 128, 0, 0);
-      constexpr uint32_t idesc_o = make_idesc_bf16(128, 64, 0, 1);  // B (= V) is MN-major
-      const uint32_t tm = __shfl_sync(0xffffffffu, tmem_base, 0);
-      const uint64_t dQ = make_smem_desc_sw128(smem_u32(sQ), 0, 1024);      // + tile * (kTileBytes >> 4)
-      const uint64_t dK = make_smem_desc_sw128(smem_u32(sK), 0, 1024);
-      const uint64_t dV = make_smem_desc_sw128(smem_u32(sV), 1024, 1024);
-      const uint64_t dP = make_smem_desc_sw128(smem_u32(sP), 0, 1024);
-      constexpr uint32_t kTileD = kTileBytes >> 4;  // descriptor address units (16 B)
-      // the single-tile tail item (always the CTA's last) belongs to one issue warp only
-      const bool skip_last = MMA2 && has_half && ((cta & 1) != t_lo);
-      const int G = (n_my - (skip_last ? 1 : 0)) * nkv;  // KV blocks this warp issues for, over all of its items
-      // All ring / item bookkeeping is incremental (no divisions on the issue path).
-      int q_it = 0, q_j = 0, q_st = 0, q_ph = 0;  // next S block to issue: item, block in item, kv stage/phase
-      // tiles this warp issues for in item `it`: its own tile(s), minus the sibling's tile of a single-tile tail item
-      auto item_tiles = [&](int it) {
-        const int mine = MMA2 ? (1 << t_lo) : 3;
-        return (has_half && it == n_my - 1) ? (mine & (1 << (cta & 1))) : mine;
-      };
-      auto issue_qk_block = [&](int gb) {
-        const int qb = q_it & 1;
-        const int tiles = item_tiles(q_it);
-        if (q_j == 0) mbar_wait(&q_full[qb], (q_it >> 1) & 1);
-        mbar_wait(&kv_full[q_st], q_ph);
-        LN3_TR(2, gb, 0);  // K of block gb landed
-        const uint64_t kd = dK + static_cast<uint32_t>(q_st) * kTileD;
+  } else if (warp >= kMmaWarp) {
+    // ------------------------------------------------------------ MMA issuers, one warp per query tile
+    // A single in-order issuing warp serialises the three tiles: tcgen05.mma issue blocks while the pipe's
+    // short queue is full, so every group of 4-6 MMAs costs its execution time plus ~150-300 cycles of wait /
+    // fence / commit latency (tools/microbench/umma_rate.cu), and with six groups per KV block P_t sat ~1800
+    // cycles in shared memory before its P V was even issued.  With one warp per tile a tile's S -> P -> O chain
+    // waits only for its own warpgroup; the three warps' MMAs interleave in the tensor pipe.
+    // The whole warp walks this code with warp-uniform values (descriptors stay in uniform registers);
+    // elect_one_sync() guards only the tcgen05 instructions.
+    const int t = warp - kMmaWarp;
+    constexpr uint32_t idesc_s = make_idesc_bf16(128, kKB, 0, 0);
+    constexpr uint32_t idesc_o = make_idesc_bf16(128, kHD, 0, 1);  // B (= V) is MN-major
+    const uint32_t tm = __shfl_sync(0xffffffffu, tmem_base, 0);
+    constexpr uint32_t kQD = kQBytes >> 4, kKVD = kKVBytes >> 4, kPD = kPBytes >> 4;  // descriptor units (16 B)
+    const uint64_t dQ = make_smem_desc_sw128(smem_u32(sQ), 0, 1024) + static_cast<uint32_t>(t) * kQD;
+    const uint64_t dK = make_smem_desc_sw128(smem_u32(sK), 0, 1024);
+    const uint64_t dV = make_smem_desc_sw128(smem_u32(sV), 1024, 1024);
+    const uint64_t dP = make_smem_desc_sw128(smem_u32(sP), 0, 1024) + static_cast<uint32_t>(t) * kPD;
+    const uint32_t tS = tm + t * kKB, tO = tm + kTmemO + t * kHD;
+
+    // cursor over the (item, block) sequence of this CTA, skipping items with an empty tile set
+    struct Cursor { int it, j, mask, st, ph, items; bool end; };
+    auto cur_init = [&](Cursor& c) {
+      c.it = -1; c.j = nkv - 1; c.mask = 0; c.st = kStages - 1; c.ph = 1; c.items = -1; c.end = false;
+    };
+    auto cur_next = [&](Cursor& c) {   // advance by one block
+      if (++c.st == kStages) c.st = 0, c.ph ^= 1;
+      if (++c.j < nkv) return;
+      c.j = 0;
+      int q0, head, batch;
+      do {
+        if (++c.it >= n_my) { c.end = true; c.mask = 0; return; }
+        c.mask = sched(c.it, q0, head, batch);
+      } while (c.mask == 0);
+      ++c.items;
+    };
+    Cursor cq, cp;   // next S block to issue / next P V block to issue
+    cur_init(cq);
+    cur_init(cp);
+    cur_next(cq);
+    cur_next(cp);
+    int n_qk = 0, n_pv = 0;   // issue counts of this tile (barrier parities)
+    int seq = 0;              // trace only
+
+    // S_t of the block under `cq` (or, when the item does not include this tile, only the ring releases)
+    auto qk_step = [&]() {
+      if (cq.j == 0) mbar_wait_hint(q_full, cq.items & 1, kWaitNs);
+      mbar_wait_hint(&k_full[cq.st], cq.ph, kWaitNs);
+      if (cq.mask >> t & 1) {
+        if (n_qk > 0) mbar_wait_hint(&s_empty[t], (n_qk - 1) & 1, kWaitNs);  // the previous S_t is in registers
+        ++n_qk;
+        tc_fence_after();
+        const uint64_t kd = dK + static_cast<uint32_t>(cq.st) * kKVD;
+        if (elect_one_sync()) {
 #pragma unroll
-        for (int t = t_lo; t < t_hi; ++t) {
-          if (!(tiles >> t & 1)) continue;
-          if (gb > 0) mbar_wait(&s_empty[t], (gb - 1) & 1);  // S_t of block gb-1 is in registers
-          tc_fence_after();
-          const uint64_t qd = dQ + static_cast<uint32_t>(qb * 2 + t) * kTileD;
-          if (elect_one_sync()) {
-#pragma unroll
-            for (int k = 0; k < kHD / 16; ++k)
-              umma_f16_ss(tm + t * 128, qd + 2 * k, kd + 2 * k, idesc_s, k != 0);
-            umma_commit(&s_full[t]);
-          }
-          __syncwarp();
-          LN3_TR(2, gb, 1 + t);  // QK_t(gb) issued
+          for (int k = 0; k < kHD / 16; ++k) umma_f16_ss(tS, dQ + 2 * k, kd + 2 * k, idesc_s, k != 0);
+          umma_commit(&s_full[t]);
+          umma_commit(&k_empty[cq.st]);
+          if (cq.j == nkv - 1) umma_commit(q_empty);
         }
-        if (++q_j == nkv) {
-          if (elect_one_sync()) umma_commit(&q_empty[qb]);  // every QK of this item has been issued
-          __syncwarp();
-          q_j = 0;
-          ++q_it;
-        }
-        if (++q_st == kKVStages) q_st = 0, q_ph ^= 1;
-      };
-      if (G > 0) issue_qk_block(0);
-      int j = 0, st = 0, pv_it = 0;
-      for (int g = 0; g < G; ++g) {
-        if (g + 1 < G) issue_qk_block(g + 1);
-        const int pv_tiles = item_tiles(pv_it);
-        const int kv_valid = (j < nkv1) ? p.Lkv - j * kKT : p.Lkv2 - (j - nkv1) * kKT;
-        const int ksteps = kv_valid >= kKT ? kKT / 16 : (kv_valid + 15) >> 4;  // P beyond is never written
-        const uint64_t vd = dV + static_cast<uint32_t>(st) * kTileD;
-#pragma unroll
-        for (int t = t_lo; t < t_hi; ++t) {
-          if (!(pv_tiles >> t & 1)) continue;
-          mbar_wait(&p_full[t], g & 1);  // P_t in smem, O_t rescaled if needed
-          LN3_TR(2, g, 3 + 2 * t);  // p_full seen
-          tc_fence_after();
-          const uint64_t pd = dP + static_cast<uint32_t>(t * 2) * kTileD;
-          if (elect_one_sync()) {
-#pragma unroll
-            for (int k = 0; k < kKT / 16; ++k)
-              if (k < ksteps) {
-                if constexpr (PTMEM)
-                  umma_f16_ts(tm + 256 + t * 64, tm + 384 + t * 64 + k * 8, vd + k * 128, idesc_o, (j | k) != 0);
-                else
-                  umma_f16_ss(tm + 256 + t * 64, pd + (k >> 2) * kTileD + (k & 3) * 2, vd + k * 128, idesc_o,
-                              (j | k) != 0);
-              }
-            umma_commit(&o_full[t]);
-          }
-          __syncwarp();
-          LN3_TR(2, g, 4 + 2 * t);  // PV_t(g) issued
-        }
-        if (elect_one_sync()) umma_commit(&kv_empty[st]);  // every MMA that read K / V of block g has been issued
         __syncwarp();
-        if (++j == nkv) j = 0, ++pv_it;
-        if (++st == kKVStages) st = 0;
-      }
-      if (skip_last) {
-        // the sibling's single-tile item: this warp issues nothing, but the K/V ring needs both warps'
-        // releases per stage (the stage's previous user must have landed first: wait kv_full, then arrive)
-        for (int jj = 0; jj < nkv; ++jj) {
-          mbar_wait(&kv_full[q_st], q_ph);
-          if (elect_one_sync()) mbar_arrive(&kv_empty[q_st]);
-          __syncwarp();
-          if (++q_st == kKVStages) q_st = 0, q_ph ^= 1;
+      } else {
+        if (elect_one_sync()) {
+          mbar_arrive(&k_empty[cq.st]);
+          if (cq.j == nkv - 1) mbar_arrive(q_empty);
         }
+        __syncwarp();
       }
+      LN3_TR3(3, seq, t);
+      cur_next(cq);
+    };
+    auto pv_step = [&]() {
+      mbar_wait_hint(&v_full[cp.st], cp.ph, kWaitNs);
+      if (cp.mask >> t & 1) {
+        const int kv_valid = (cp.j < nkv1) ? p.Lkv - cp.j * kKB : p.Lkv2 - (cp.j - nkv1) * kKB;
+        const int ksteps = kv_valid >= kKB ? kKB / 16 : (kv_valid + 15) >> 4;  // P beyond is never written
+        const uint64_t vd = dV + static_cast<uint32_t>(cp.st) * kKVD;
+        mbar_wait_hint(&p_full[t], n_pv & 1, kWaitNs);  // P_t in smem, O_t rescaled if needed
+        ++n_pv;
+        LN3_TR3(3, seq, 3 + 2 * t);
+        tc_fence_after();
+        if (elect_one_sync()) {
+#pragma unroll
+          for (int k = 0; k < kKB / 16; ++k)
+            if (k < ksteps)
+              umma_f16_ss(tO, dP + (k >> 2) * kQD + (k & 3) * 2, vd + k * 128, idesc_o, (cp.j | k) != 0);
+          umma_commit(&o_full[t]);
+          umma_commit(&v_empty[cp.st]);
+        }
+        __syncwarp();
+        LN3_TR3(3, seq, 4 + 2 * t);
+      } else {
+        if (elect_one_sync()) mbar_arrive(&v_empty[cp.st]);
+        __syncwarp();
+      }
+      ++seq;
+      cur_next(cp);
+    };
+    // S(0) and S(1) up front, then per block: P V(g), and S(g+2) as soon as the warpgroup has S(g+1) in registers
+    for (int pre = 0; pre < 2 && !cq.end; ++pre) qk_step();
+    while (!cp.end) {
+      pv_step();
+      if (!cq.end) qk_step();
     }
-  } else if (!SPLIT && warp < 8) {
+  } else {
     // ------------------------------------------------------------ softmax warpgroups
     const int t = warp >> 2;
     const int row = tid & 127;  // TMEM lane
     const uint32_t lane_off = static_cast<uint32_t>((warp & 3) * 32) << 16;
-    const uint32_t tS = tmem_base + t * 128 + lane_off;
-    const uint32_t tO = tmem_base + 256 + t * 64 + lane_off;
-    const uint32_t tP = tmem_base + 384 + t * 64 + lane_off;   // PTMEM: P_t as packed bf16 pairs
-    const uint32_t p_row = smem_u32(sP + t * 2 * kTileBytes) + row * 128;
+    const uint32_t tS = tmem_base + t * kKB + lane_off;
+    const uint32_t tO = tmem_base + kTmemO + t * kHD + lane_off;
+    uint8_t* sPt = sP + t * kPBytes;
+    const uint32_t p_row = smem_u32(sPt) + row * 128;
     const int swz = row & 7;
-    int g = 0;
+    int g = 0;    // blocks of items this tile took part in (per-tile barrier parities)
     bool o_store_pending = false;  // thread 0 of the group: a bulk store may still be reading P_t's smem
-    // XU baton: the two warpgroups take turns in the exponential phase (named barriers 1 + t, 256
-    // participants = 128 waiting + 128 arriving).  Left alone they fall into lock-step -- both in the
-    // MUFU-bound phase together, then both idle on the tensor core -- and the XU pipe sits at ~45 %.
-    if (PINGPONG && t == 1) named_bar_arrive(1, 256);  // warpgroup 0 goes first
     for (int it = 0; it < n_my; ++it) {
-      int w, mask, q0, head, batch;
-      sched(it, w, mask);
-      if (!(mask >> t & 1)) break;  // the sibling tile's single-tile tail item (always last)
-      item_coords(w, q0, head, batch);
+      int q0, head, batch;
+      const int mask = sched(it, q0, head, batch);
+      if (!(mask >> t & 1)) continue;
       float m_ref = -INFINITY, l_run = 0.f;
       for (int j = 0; j < nkv; ++j, ++g) {
-        const int kv_valid = (j < nkv1) ? p.Lkv - j * kKT : p.Lkv2 - (j - nkv1) * kKT;  // >= 1
-        if (row == 0) LN3_TR(t, g, 0);  // start waiting for S
-        mbar_wait(&s_full[t], g & 1);
-        if (row == 0) LN3_TR(t, g, 1);  // S ready
+        const int kv_valid = (j < nkv1) ? p.Lkv - j * kKB : p.Lkv2 - (j - nkv1) * kKB;  // >= 1
+        if (row == 0) LN3_TR3(t, g, 0);  // start waiting for S
+        mbar_wait_hint(&s_full[t], g & 1, kWaitNs);
+        if (row == 0) LN3_TR3(t, g, 1);  // S ready
         tc_fence_after();
-        uint32_t s[128];
+        uint32_t s[kKB];
         tmem_ld_32x32(tS + 0, s);
         tmem_ld_32x32(tS + 32, s + 32);
         tmem_ld_32x32(tS + 64, s + 64);
-        tmem_ld_32x32(tS + 96, s + 96);
         tmem_ld_wait();
-        if (row == 0) LN3_TR(t, g, 2);  // S in registers
+        if (row == 0) LN3_TR3(t, g, 2);  // S in registers
         tc_fence_before();
-        mbar_arrive(&s_empty[t]);  // the tensor core may overwrite S_t with the next block now
-        if (kv_valid < kKT) {
+        // one arrival per warp: 128 per-thread arrivals are 128 serialised barrier updates on the MIO queue the
+        // exponentials of the other warpgroups are competing for
+        __syncwarp();
+        if ((tid & 31) == 0) mbar_arrive(&s_empty[t]);  // the tensor core may overwrite S_t with the next block now
+        if (kv_valid < kKB) {
 #pragma unroll
-          for (int i = 0; i < 128; ++i)
+          for (int i = 0; i < kKB; ++i)
             if (i >= kv_valid) s[i] = 0xff800000u;  // -inf
         }
-        const int c_end = kv_valid >= kKT ? kKT : (kv_valid + 15) & ~15;  // = 16 * PV k-steps
-        // four independent 3-input max chains (a single chain is 64 dependent FMNMX3 deep)
-        float mq[4];
+        if (p.causal) {   // (first K/V source only; every row keeps key 0, so block 0 is never fully masked)
+          const int lim = q0 + t * kQT + row - j * kKB;   // columns i > lim are in the future of this row
 #pragma unroll
-        for (int a = 0; a < 4; ++a) {
-          const int b0 = 32 * a;
-          mq[a] = fmax3(__uint_as_float(s[b0]), __uint_as_float(s[b0 + 1]), __uint_as_float(s[b0 + 2]));
+          for (int i = 0; i < kKB; ++i)
+            if (i > lim) s[i] = 0xff800000u;
         }
-#pragma unroll
-        for (int i = 3; i < 31; i += 2) {
-#pragma unroll
-          for (int a = 0; a < 4; ++a)
-            mq[a] = fmax3(mq[a], __uint_as_float(s[32 * a + i]), __uint_as_float(s[32 * a + i + 1]));
-        }
-        const float mx = fmax3(fmax3(mq[0], mq[1], mq[2]), mq[3],
-                               fmax3(__uint_as_float(s[31]), __uint_as_float(s[63]),
-                                     fmaxf(__uint_as_float(s[95]), __uint_as_float(s[127]))));
-        const float m_cand = mx * p.scale_log2;
+        const int c_end = kv_valid >= kKB ? kKB : (kv_valid + 15) & ~15;  // = 16 * PV k-steps
+        // Only the first block of an item pays a separate max pass.  Later blocks exponentiate against the running
+        // reference straight away and track their own maximum INSIDE the exponential loop (FMNMX on the ALU pipe, in
+        // the issue slots the XU-bound loop leaves free); if the block then turns out to exceed the reference by more
+        // than the lazy-rescale threshold -- rare: the threshold is 2^8 -- the block is redone against the new maximum.
         float alpha = 1.f;
         bool need = false;
         if (j == 0) {
-          m_ref = m_cand;
-        } else if (m_cand > m_ref + kRescaleThreshold) {
-          need = true;
-          alpha = fast_exp2(m_ref - m_cand);
-          m_ref = m_cand;
-          l_run *= alpha;
+          // three independent 3-input max chains
+          float mq[3];
+#pragma unroll
+          for (int a = 0; a < 3; ++a) {
+            const int b0 = 32 * a;
+            mq[a] = fmax3(__uint_as_float(s[b0]), __uint_as_float(s[b0 + 1]), __uint_as_float(s[b0 + 2]));
+          }
+#pragma unroll
+          for (int i = 3; i < 31; i += 2) {
+#pragma unroll
+            for (int a = 0; a < 3; ++a)
+              mq[a] = fmax3(mq[a], __uint_as_float(s[32 * a + i]), __uint_as_float(s[32 * a + i + 1]));
+          }
+          const float mx = fmax3(fmax3(mq[0], mq[1], mq[2]), __uint_as_float(s[31]),
+                                 fmaxf(__uint_as_float(s[63]), __uint_as_float(s[95])));
+          m_ref = mx * p.scale_log2;
         }
-        // P_t (smem) is still being read by P_t V of the previous block until o_full fires; S of this
-        // block was issued ahead of that MMA, so s_full alone no longer orders the two.
-        if (row == 0) LN3_TR(t, g, 3);  // max done
+        if (row == 0) LN3_TR3(t, g, 3);  // max done
         if (j == 0 && g > 0) {  // previous item's O tile left this buffer?  (long done; one barrier per item)
           if (row == 0 && o_store_pending) tma_store_wait_read();
-          named_bar_sync(3 + t, 128);
+          named_bar_sync(3 + t, kQT);
         }
-        if (g > 0) mbar_wait(&o_full[t], (g - 1) & 1);
-        if (row == 0) LN3_TR(t, g, 4);  // O of previous block complete
-        if (PINGPONG) named_bar_sync(1 + t, 256);
-        if (row == 0) LN3_TR(t, g, 5);  // baton
-        // FULL blocks: one straight-line region of 128 exponentials (the scheduler interleaves MUFU,
-        // polynomial and st.shared across chunks); ragged last block: stop at c_end.
+        // P_t (smem) is read by P_t V of the previous block until o_full fires
+        if (g > 0) mbar_wait_hint(&o_full[t], (g - 1) & 1, kWaitNs);
+        if (row == 0) LN3_TR3(t, g, 4);  // O of previous block complete
         float rs = 0.f;
-        // FULL blocks: one straight-line region of 128 exponentials (the scheduler interleaves MUFU and
-        // st.shared across chunks); ragged last block: stop at c_end.  (Packed FFMA2/FADD2 here measured
-        // slower: the 64-bit register pairs push the 168-register budget into spills.)
+        float mb[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};   // running maxima of this block's scores
         auto exp_store = [&](auto full_tag) {
           constexpr bool FULL = decltype(full_tag)::value;
 #pragma unroll
-          for (int c = 0; c < 128; c += 8) {
+          for (int c = 0; c < kKB; c += 8) {
             if (!FULL && c >= c_end) break;
             float e[8];
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
-              const float x = fmaf(__uint_as_float(s[c + i]), p.scale_log2, -m_ref);
-              e[i] = (i < kPolyPer8) ? exp2_poly(x) : fast_exp2(x);
+              e[i] = fast_exp2(fmaf(__uint_as_float(s[c + i]), p.scale_log2, -m_ref));
+              mb[i & 3] = fmaxf(mb[i & 3], __uint_as_float(s[c + i]));
             }
             rs += ((e[0] + e[1]) + (e[2] + e[3])) + ((e[4] + e[5]) + (e[6] + e[7]));
-            if constexpr (PTMEM) {
-              // in place: the score registers of this chunk become the packed probabilities; every 64 columns
-              // (32 packed words) go to tensor memory with one tcgen05.st
-              s[c / 2 + 0] = pack_bf16x2(e[0], e[1]);
-              s[c / 2 + 1] = pack_bf16x2(e[2], e[3]);
-              s[c / 2 + 2] = pack_bf16x2(e[4], e[5]);
-              s[c / 2 + 3] = pack_bf16x2(e[6], e[7]);
-              if ((c & 63) == 56) tmem_st_32x32(tP + (c >> 6) * 32, s + (c >> 6) * 32);
-            } else {
-              const uint32_t addr = p_row + (c >> 6) * kTileBytes + ((((c & 63) >> 3) ^ swz) << 4);
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(pack_bf16x2(e[0], e[1])),
-                           "r"(pack_bf16x2(e[2], e[3])), "r"(pack_bf16x2(e[4], e[5])),
-                           "r"(pack_bf16x2(e[6], e[7]))
-                           : "memory");
-            }
-          }
-          if constexpr (PTMEM && !FULL) {  // ragged block: flush the half that the loop left unfinished
-            if ((c_end & 63) != 0) {
-              if (c_end < 64) tmem_st_32x32(tP, s);
-              else tmem_st_32x32(tP + 32, s + 32);
-            }
+            const uint32_t addr = p_row + (c >> 6) * kQBytes + ((((c & 63) >> 3) ^ swz) << 4);
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(pack_bf16x2(e[0], e[1])),
+                         "r"(pack_bf16x2(e[2], e[3])), "r"(pack_bf16x2(e[4], e[5])),
+                         "r"(pack_bf16x2(e[6], e[7]))
+                         : "memory");
           }
         };
-        if (kv_valid >= kKT) exp_store(std::true_type{});
+        if (kv_valid >= kKB) exp_store(std::true_type{});
         else exp_store(std::false_type{});
-        if (row == 0) LN3_TR(t, g, 6);  // exponentials done
-        if (PINGPONG) named_bar_arrive(2 - t, 256);
+        if (j > 0) {
+          const float m_cand = fmaxf(fmaxf(mb[0], mb[1]), fmaxf(mb[2], mb[3])) * p.scale_log2;
+          need = m_cand > m_ref + kRescaleThreshold;
+          if (__any_sync(0xffffffffu, need)) {
+            // redo the block against the new reference (rows without `need` recompute the same values)
+            if (need) {
+              alpha = fast_exp2(m_ref - m_cand);
+              m_ref = m_cand;
+              l_run *= alpha;
+            }
+            rs = 0.f;
+            if (kv_valid >= kKB) exp_store(std::true_type{});
+            else exp_store(std::false_type{});
+          }
+        }
+        if (row == 0) LN3_TR3(t, g, 6);  // exponentials done
         l_run += rs;
         if (j > 0 && __any_sync(0xffffffffu, need)) {
           // O_t of the previous block is complete (o_full waited above): rescale it in place
@@ -460,19 +433,18 @@ fmha_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
           }
           tmem_st_wait();
         }
-        if constexpr (PTMEM) tmem_st_wait();          // P (tcgen05.st) complete
-        else fence_proxy_async_smem();                // P (generic-proxy stores) -> visible to the tensor core
+        fence_proxy_async_smem();  // P (generic-proxy stores) -> visible to the tensor core
         tc_fence_before();
-        mbar_arrive(&p_full[t]);
-        if (row == 0) LN3_TR(t, g, 7);  // P handed to the tensor core
+        __syncwarp();
+        if ((tid & 31) == 0) mbar_arrive(&p_full[t]);
+        if (row == 0) LN3_TR3(t, g, 7);  // P handed to the tensor core
       }
-      if (row == 0) LN3_TR(t, g - 1, 8);   // epilogue: start waiting for the last P V
-      mbar_wait(&o_full[t], (g - 1) & 1);
-      if (row == 0) LN3_TR(t, g - 1, 9);   // O complete
+      if (row == 0) LN3_TR3(t, g - 1, 8);   // epilogue: start waiting for the last P V
+      mbar_wait_hint(&o_full[t], (g - 1) & 1, kWaitNs);
+      if (row == 0) LN3_TR3(t, g - 1, 9);   // O complete
       tc_fence_after();
       const float inv = 1.f / l_run;
-      // O_t -> bf16 -> this tile's (now idle) P buffer in the 128B-swizzled TMA layout -> one bulk tensor
-      // store per tile.  (Per-thread row stores touched 32 lines per instruction: ~2000 cycles per item.)
+      // O_t -> bf16 -> this tile's (now idle) P buffer in the 128B-swizzled TMA layout -> one bulk tensor store
 #pragma unroll
       for (int c = 0; c < kHD; c += 32) {
         uint32_t v[32];
@@ -491,172 +463,21 @@ fmha_fwd_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constan
       }
       fence_proxy_async_smem();
       tc_fence_before();  // the TMEM reads above precede the next item's first P_t V (accumulate = 0)
-      named_bar_sync(3 + t, 128);
+      named_bar_sync(3 + t, kQT);
       if (row == 0) {
-        tma_store_3d(sP + t * 2 * kTileBytes, &tmap_o, head * kHD, q0 + t * kQT, batch);
+        tma_store_3d(sPt, &tmap_o, head * kHD, q0 + t * kQT, batch);
         tma_store_commit();
         o_store_pending = true;
       }
-      if (row == 0) LN3_TR(t, g - 1, 10);  // O stored
+      if (row == 0) LN3_TR3(t, g - 1, 10);  // O stored
     }
-    if (PINGPONG && t == 0) named_bar_sync(1, 256);  // consume warpgroup 1's last hand-over
     if (row == 0 && o_store_pending) tma_store_wait_all();  // smem must outlive the bulk store
-  } else if (SPLIT && warp < 16) {
-    // ------------------------------------------------------------ softmax, two warpgroups per tile
-    const int t = warp >> 3;            // query tile
-    const int h = (warp >> 2) & 1;      // column half of every 128-column score block (= P atom)
-    const int row = (warp & 3) * 32 + (tid & 31);  // TMEM lane
-    const uint32_t lane_off = static_cast<uint32_t>((warp & 3) * 32) << 16;
-    const uint32_t tS = tmem_base + t * 128 + h * 64 + lane_off;
-    const uint32_t tO = tmem_base + 256 + t * 64 + lane_off;
-    const uint32_t tX = tmem_base + 384 + t * 8 + lane_off;   // exchange: [parity][half] max, [4 + half] sum
-    const uint32_t p_row = smem_u32(sP + (t * 2 + h) * kTileBytes) + row * 128;
-    const uint32_t o_row = smem_u32(sP + t * 2 * kTileBytes) + row * 128;
-    const int swz = row & 7;
-    int g = 0;
-    bool o_store_pending = false;
-    for (int w = blockIdx.x; w < nitems; w += gridDim.x) {
-      int q0, head, batch;
-      item_coords(w, q0, head, batch);
-      float m_ref = -INFINITY, l_run = 0.f;
-      for (int j = 0; j < nkv; ++j, ++g) {
-        const int kv_valid = (j < nkv1) ? p.Lkv - j * kKT : p.Lkv2 - (j - nkv1) * kKT;  // >= 1
-        const int my_valid = kv_valid - h * 64;                                          // of my 64 columns (may be <= 0)
-        mbar_wait(&s_full[t], g & 1);
-        tc_fence_after();
-        uint32_t s[64];
-        tmem_ld_32x32(tS + 0, s);
-        tmem_ld_32x32(tS + 32, s + 32);
-        tmem_ld_wait();
-        tc_fence_before();
-        mbar_arrive(&s_empty[t]);  // the tensor core may overwrite S_t with the next block now
-        if (my_valid < 64) {
-#pragma unroll
-          for (int i = 0; i < 64; ++i)
-            if (i >= my_valid) s[i] = 0xff800000u;  // -inf
-        }
-        float mq[2];
-#pragma unroll
-        for (int a = 0; a < 2; ++a)
-          mq[a] = fmax3(__uint_as_float(s[32 * a]), __uint_as_float(s[32 * a + 1]), __uint_as_float(s[32 * a + 2]));
-#pragma unroll
-        for (int i = 3; i < 31; i += 2) {
-#pragma unroll
-          for (int a = 0; a < 2; ++a)
-            mq[a] = fmax3(mq[a], __uint_as_float(s[32 * a + i]), __uint_as_float(s[32 * a + i + 1]));
-        }
-        float mx = fmax3(mq[0], mq[1], fmaxf(__uint_as_float(s[31]), __uint_as_float(s[63])));
-        // the row's block maximum is the max over both halves: swap through TMEM (parity double buffer,
-        // one 256-thread named barrier per block)
-        tmem_st_32x1(tX + (g & 1) * 2 + h, __float_as_uint(mx));
-        tmem_st_wait();
-        tc_fence_before();
-        named_bar_sync(1 + t, 256);
-        tc_fence_after();
-        mx = fmaxf(mx, __uint_as_float(tmem_ld_32x1(tX + (g & 1) * 2 + (1 - h))));
-        tmem_ld_wait();
-        const float m_cand = mx * p.scale_log2;
-        float alpha = 1.f;
-        bool need = false;
-        if (j == 0) {
-          m_ref = m_cand;
-        } else if (m_cand > m_ref + kRescaleThreshold) {
-          need = true;
-          alpha = fast_exp2(m_ref - m_cand);
-          m_ref = m_cand;
-          l_run *= alpha;
-        }
-        if (j == 0 && g > 0) {  // previous item's O tile left the P buffer? (one barrier per item)
-          if (h == 0 && row == 0 && o_store_pending) tma_store_wait_read();
-          named_bar_sync(3 + t, 256);
-        }
-        // my P atom is read by k-steps 4h .. 4h+3 of the previous P_t V: wait for the whole MMA
-        if (g > 0) mbar_wait(&o_full[t], (g - 1) & 1);
-        const int c_end = my_valid >= 64 ? 64 : (my_valid <= 0 ? 0 : (my_valid + 15) & ~15);
-        float rs = 0.f;
-        auto exp_store = [&](auto full_tag) {
-          constexpr bool FULL = decltype(full_tag)::value;
-#pragma unroll
-          for (int c = 0; c < 64; c += 8) {
-            if (!FULL && c >= c_end) break;
-            float e[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const float x = fmaf(__uint_as_float(s[c + i]), p.scale_log2, -m_ref);
-              e[i] = (i < kPolyPer8) ? exp2_poly(x) : fast_exp2(x);
-            }
-            rs += ((e[0] + e[1]) + (e[2] + e[3])) + ((e[4] + e[5]) + (e[6] + e[7]));
-            const uint32_t addr = p_row + (((c >> 3) ^ swz) << 4);
-            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(pack_bf16x2(e[0], e[1])),
-                         "r"(pack_bf16x2(e[2], e[3])), "r"(pack_bf16x2(e[4], e[5])),
-                         "r"(pack_bf16x2(e[6], e[7]))
-                         : "memory");
-          }
-        };
-        if (my_valid >= 64) exp_store(std::true_type{});
-        else exp_store(std::false_type{});
-        l_run += rs;
-        if (j > 0 && __any_sync(0xffffffffu, need)) {
-          // both halves took the same decision (same combined maximum); half 0 rescales O_t in place
-          tc_fence_after();
-          if (h == 0) {
-#pragma unroll
-            for (int c = 0; c < kHD; c += 32) {
-              uint32_t v[32];
-              tmem_ld_32x32(tO + c, v);
-              tmem_ld_wait();
-#pragma unroll
-              for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(__uint_as_float(v[i]) * alpha);
-              tmem_st_32x32(tO + c, v);
-            }
-            tmem_st_wait();
-          }
-        }
-        fence_proxy_async_smem();  // P (generic-proxy stores) -> visible to the tensor core
-        tc_fence_before();
-        mbar_arrive(&p_full[t]);
-      }
-      // ---- epilogue: total row sum = both halves, each half normalises and stores 32 of the 64 O columns
-      tmem_st_32x1(tX + 4 + h, __float_as_uint(l_run));
-      tmem_st_wait();
-      tc_fence_before();
-      mbar_wait(&o_full[t], (g - 1) & 1);
-      named_bar_sync(1 + t, 256);
-      tc_fence_after();
-      const float l_tot = l_run + __uint_as_float(tmem_ld_32x1(tX + 4 + (1 - h)));
-      tmem_ld_wait();
-      const float inv = 1.f / l_tot;
-      {
-        uint32_t v[32];
-        tmem_ld_32x32(tO + h * 32, v);
-        tmem_ld_wait();
-#pragma unroll
-        for (int i = 0; i < 32; i += 8) {
-          const uint32_t addr = o_row + ((((h * 32 + i) >> 3) ^ swz) << 4);
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr),
-                       "r"(pack_bf16x2(__uint_as_float(v[i]) * inv, __uint_as_float(v[i + 1]) * inv)),
-                       "r"(pack_bf16x2(__uint_as_float(v[i + 2]) * inv, __uint_as_float(v[i + 3]) * inv)),
-                       "r"(pack_bf16x2(__uint_as_float(v[i + 4]) * inv, __uint_as_float(v[i + 5]) * inv)),
-                       "r"(pack_bf16x2(__uint_as_float(v[i + 6]) * inv, __uint_as_float(v[i + 7]) * inv))
-                       : "memory");
-        }
-      }
-      fence_proxy_async_smem();
-      tc_fence_before();  // the TMEM reads above precede the next item's first P_t V (accumulate = 0)
-      named_bar_sync(3 + t, 256);
-      if (h == 0 && row == 0) {
-        tma_store_3d(sP + t * 2 * kTileBytes, &tmap_o, head * kHD, q0 + t * kQT, batch);
-        tma_store_commit();
-        o_store_pending = true;
-      }
-    }
-    if (h == 0 && row == 0 && o_store_pending) tma_store_wait_all();  // smem must outlive the bulk store
   }
 
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  if (warp == kMmaWarp) tmem_dealloc(tmem_base, kFmhaTmemCols);
+  if (warp == kMmaWarp) tmem_dealloc(tmem_base, kTmemCols);
 }
 
 int fmha_fwd(const ln3_fmha_args* a, cudaStream_t stream) {
@@ -668,94 +489,31 @@ int fmha_fwd(const ln3_fmha_args* a, cudaStream_t stream) {
   if ((reinterpret_cast<uintptr_t>(a->q) | reinterpret_cast<uintptr_t>(a->k) |
        reinterpret_cast<uintptr_t>(a->v) | reinterpret_cast<uintptr_t>(a->out)) & 15)
     return set_error(LN3_EINVAL, "fmha: pointers must be 16-byte aligned");
-  // LN3_FMHA_KERNEL: 3 (default) = three-warpgroup rota kernel (attention3_tcgen05.cu), 2 = the two-warpgroup
-  // kernel of this file.  LN3_FMHA_ROTA=1 switches the exponential-phase rota on (measured 2 % slower), LN3_FMHA_POLY=2 moves 2 of 8 exponentials to the FMA pipe.
-  static const int kernel3 = [] {
-    const char* kv = getenv("LN3_FMHA_KERNEL");
-    if (kv && atoi(kv) == 2) return -1;
-    const char* ro = getenv("LN3_FMHA_ROTA");
-    const char* po = getenv("LN3_FMHA_POLY");
-    const char* lz = getenv("LN3_FMHA_LAZYMAX");
-    const char* ch = getenv("LN3_FMHA_CHAIN");
-    const bool plain = !(ro && atoi(ro) != 0) && !(po && atoi(po) == 2) && !(ch && atoi(ch) != 0);
-    // default: block maximum tracked inside the exponential loop (82.3 -> 80.3 us); LN3_FMHA_LAZYMAX=0 or any of the
-    // other knobs selects the separate max pass
-    if (plain && !(lz && atoi(lz) == 0)) return 9;
-    if (lz && atoi(lz) == 2) return 10;   // LN3_FMHA_LAZYMAX=2: lazy maximum + packed 2-of-8 polynomial exponentials
-    const int chain = (ch && atoi(ch) != 0) ? 4 : 0;   // LN3_FMHA_CHAIN=1: dependency-chained exponential loop
-    if (chain) return ((ro && atoi(ro) != 0) ? 0 : 1) | chain;
-    return ((ro && atoi(ro) != 0) ? 0 : 1) | ((po && atoi(po) == 2) ? 2 : 0);   // bit 0 = rota OFF (default)
-  }();
   if (a->causal && (a->k2 != nullptr || a->v2 != nullptr))
     return set_error(LN3_EINVAL, "fmha: causal attention takes a single K/V source");
-  if (a->causal && kernel3 < 0) return set_error(LN3_EUNSUPPORTED, "fmha: the two-warpgroup kernel has no causal mask");
-  if (kernel3 >= 0) {
-    if (a->k2 != nullptr || a->v2 != nullptr) {
-      if (!a->k2 || !a->v2 || a->Lkv2 <= 0) return set_error(LN3_EINVAL, "fmha: k2/v2/Lkv2 must be given together");
-      if ((a->k2_ld | a->v2_ld | a->k2_bs | a->v2_bs) % 8 ||
-          ((reinterpret_cast<uintptr_t>(a->k2) | reinterpret_cast<uintptr_t>(a->v2)) & 15))
-        return set_error(LN3_EINVAL, "fmha: k2/v2 alignment");
-    }
-    return fmha3_launch(a, kernel3, stream);
-  }
-  // tuning knobs, read once: LN3_FMHA_POLY = exponentials per 8 on the FMA pipe (0, 2, 3, 4);
-  // LN3_FMHA_PINGPONG = 1 enables the XU baton between the two softmax warpgroups (measured: no gain)
-  static const int variant = [] {   // environment knobs: device-independent, read once (thread-safe static init)
-    const char* ev = getenv("LN3_FMHA_POLY");
-    int v = ev ? atoi(ev) : kPolyPer8Default;
-    if (v != 0 && v != 2 && v != 3 && v != 4) v = kPolyPer8Default;
-    const char* pp = getenv("LN3_FMHA_PINGPONG");
-    const int ping = (pp && atoi(pp) != 0) ? 1 : 0;
-    // LN3_FMHA_SPLIT = 1: 16 softmax warps, each tile's score columns split over two warpgroups
-    const char* sp = getenv("LN3_FMHA_SPLIT");
-    const int split = (sp && atoi(sp) != 0) ? 1 : 0;
-    // LN3_FMHA_PTMEM = 1: P through tensor memory (TMEM A operand of P V)
-    const char* pt = getenv("LN3_FMHA_PTMEM");
-    const int ptmem = (pt && atoi(pt) != 0) ? 1 : 0;
-    // LN3_FMHA_MMA2 = 1: one MMA issue warp per query tile (measured slower: the second polling warp takes issue
-    // slots from the softmax warps of its scheduler -- 85 vs 77 us at the DiT-L/2 self-attention shape)
-    const char* m2 = getenv("LN3_FMHA_MMA2");
-    const int mma2 = (m2 && atoi(m2) != 0) ? 1 : 0;
-    if (split) return 100 + (v == 2 ? 2 : 0);
-    if (ptmem) return 200;
-    if (mma2 && !ping) return 300 + v;
-    return v * 2 + ping;
-  }();
-  static DeviceOnce once;   // the shared-memory opt-in is per device
-  if (int rc = once.run([] {
-        cudaError_t e = cudaSuccess;
-        auto set = [&](auto* k) {
-          if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, kFmhaSmem);
-        };
-        set(fmha_fwd_kernel<0, false>); set(fmha_fwd_kernel<0, true>);
-        set(fmha_fwd_kernel<2, false>); set(fmha_fwd_kernel<2, true>);
-        set(fmha_fwd_kernel<3, false>); set(fmha_fwd_kernel<3, true>);
-        set(fmha_fwd_kernel<4, false>); set(fmha_fwd_kernel<4, true>);
-        set(fmha_fwd_kernel<0, false, true>); set(fmha_fwd_kernel<2, false, true>);
-        set(fmha_fwd_kernel<0, false, false, true>);
-        set(fmha_fwd_kernel<0, false, false, false, true>); set(fmha_fwd_kernel<2, false, false, false, true>);
-        set(fmha_fwd_kernel<3, false, false, false, true>); set(fmha_fwd_kernel<4, false, false, false, true>);
-        return e == cudaSuccess ? LN3_OK : set_error(LN3_ECUDA, "fmha: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-      }))
-    return rc;
   if (a->k2 != nullptr || a->v2 != nullptr) {
     if (!a->k2 || !a->v2 || a->Lkv2 <= 0) return set_error(LN3_EINVAL, "fmha: k2/v2/Lkv2 must be given together");
-    if (a->Lkv % kKT != 0) return set_error(LN3_EINVAL, "fmha: Lkv must be a multiple of 128 with a second K/V source");
     if ((a->k2_ld | a->v2_ld | a->k2_bs | a->v2_bs) % 8 ||
         ((reinterpret_cast<uintptr_t>(a->k2) | reinterpret_cast<uintptr_t>(a->v2)) & 15))
       return set_error(LN3_EINVAL, "fmha: k2/v2 alignment");
   }
+  static DeviceOnce once;   // the shared-memory opt-in is per device
+  if (int rc = once.run([] {
+        cudaError_t e = cudaFuncSetAttribute(fmha_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+        return e == cudaSuccess ? LN3_OK : set_error(LN3_ECUDA, "fmha: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+      }))
+    return rc;
+  const bool two = a->k2 != nullptr;
   CUtensorMap tq, tk, tv, tk2, tv2, to;
   int rc;
   const long long cols = static_cast<long long>(a->H) * kHD;
   if ((rc = make_tmap_3d_bf16(&tq, a->q, cols, a->Lq, a->B, a->q_ld, a->q_bs, kHD, kQT))) return rc;
-  if ((rc = make_tmap_3d_bf16(&tk, a->k, cols, a->Lkv, a->B, a->k_ld, a->k_bs, kHD, kKT))) return rc;
-  if ((rc = make_tmap_3d_bf16(&tv, a->v, cols, a->Lkv, a->B, a->v_ld, a->v_bs, kHD, kKT))) return rc;
+  if ((rc = make_tmap_3d_bf16(&tk, a->k, cols, a->Lkv, a->B, a->k_ld, a->k_bs, kHD, kKB))) return rc;
+  if ((rc = make_tmap_3d_bf16(&tv, a->v, cols, a->Lkv, a->B, a->v_ld, a->v_bs, kHD, kKB))) return rc;
   if ((rc = make_tmap_3d_bf16(&to, a->out, cols, a->Lq, a->B, a->o_ld, a->o_bs, kHD, kQT))) return rc;
-  const bool two = a->k2 != nullptr;
   if (two) {
-    if ((rc = make_tmap_3d_bf16(&tk2, a->k2, cols, a->Lkv2, a->B, a->k2_ld, a->k2_bs, kHD, kKT))) return rc;
-    if ((rc = make_tmap_3d_bf16(&tv2, a->v2, cols, a->Lkv2, a->B, a->v2_ld, a->v2_bs, kHD, kKT))) return rc;
+    if ((rc = make_tmap_3d_bf16(&tk2, a->k2, cols, a->Lkv2, a->B, a->k2_ld, a->k2_bs, kHD, kKB))) return rc;
+    if ((rc = make_tmap_3d_bf16(&tv2, a->v2, cols, a->Lkv2, a->B, a->v2_ld, a->v2_bs, kHD, kKB))) return rc;
   } else {
     tk2 = tk;
     tv2 = tv;
@@ -765,44 +523,26 @@ int fmha_fwd(const ln3_fmha_args* a, cudaStream_t stream) {
   p.Lkv = a->Lkv;
   p.Lkv2 = two ? a->Lkv2 : 0;
   p.scale_log2 = a->scale * 1.4426950408889634f;
+  p.causal = a->causal ? 1 : 0;
   p.B = a->B;
   p.H = a->H;
-  p.nq = (a->Lq + 2 * kQT - 1) / (2 * kQT);
+  p.nq = (a->Lq + kNT * kQT - 1) / (kNT * kQT);
   p.rcp_nq = 1.0f / static_cast<float>(p.nq);
   p.rcp_H = 1.0f / static_cast<float>(p.H);
   const long long nitems = static_cast<long long>(p.B) * p.H * p.nq;
-  if (nitems >= (1 << 20)) return set_error(LN3_EUNSUPPORTED, "fmha: more than 2^20 (batch, head, 256-row) work items");
+  if (nitems >= (1 << 20)) return set_error(LN3_EUNSUPPORTED, "fmha: more than 2^20 (batch, head, 384-row) work items");
   const int sms = device_sm_count();
   const int grid = static_cast<int>(nitems < sms ? nitems : sms);
   p.full_items = static_cast<int>(nitems);
   p.n_split = 0;
-  if (variant >= 300 || (variant < 100 && (variant & 1) == 0)) {
-    // tail schedule: the last, partial round as single-tile items on twice as many SMs (each warpgroup then has
-    // the SM's XU pipe to itself) when they fit.  LN3_FMHA_TAIL=0 disables.
-    static const bool tail = !(getenv("LN3_FMHA_TAIL") && atoi(getenv("LN3_FMHA_TAIL")) == 0);
-    const int rem = static_cast<int>(nitems % grid);
-    if (tail && nitems > grid && rem > 0 && 2 * rem <= grid) {
-      p.full_items = static_cast<int>(nitems) - rem;
-      p.n_split = rem;
-    }
+  // tail schedule: the last, partial round as (2 tiles | 1 tile) halves on twice as many SMs when they fit
+  const int rem = static_cast<int>(nitems % grid);
+  if (nitems > grid && rem > 0 && 2 * rem <= grid) {
+    p.full_items = static_cast<int>(nitems) - rem;
+    p.n_split = rem;
   }
-  cudaError_t le = cudaSuccess;
-  switch (variant) {
-#define LN3_FMHA_CASE(P, G) \
-  case (P) * 2 + (G): le = launch_pdl(fmha_fwd_kernel<P, (G) != 0>, dim3(grid), dim3(kFmhaThreads), kFmhaSmem, stream, tq, tk, tv, tk2, tv2, to, p); break;
-    LN3_FMHA_CASE(0, 0) LN3_FMHA_CASE(0, 1) LN3_FMHA_CASE(2, 0) LN3_FMHA_CASE(2, 1)
-    LN3_FMHA_CASE(3, 0) LN3_FMHA_CASE(3, 1) LN3_FMHA_CASE(4, 0) LN3_FMHA_CASE(4, 1)
-#undef LN3_FMHA_CASE
-    case 100: le = launch_pdl(fmha_fwd_kernel<0, false, true>, dim3(grid), dim3(fmha_threads<true>()), kFmhaSmem, stream, tq, tk, tv, tk2, tv2, to, p); break;
-    case 200: le = launch_pdl(fmha_fwd_kernel<0, false, false, true>, dim3(grid), dim3(kFmhaThreads), kFmhaSmem, stream, tq, tk, tv, tk2, tv2, to, p); break;
-    case 102: le = launch_pdl(fmha_fwd_kernel<2, false, true>, dim3(grid), dim3(fmha_threads<true>()), kFmhaSmem, stream, tq, tk, tv, tk2, tv2, to, p); break;
-#define LN3_FMHA_CASE2(P) \
-  case 300 + (P): le = launch_pdl(fmha_fwd_kernel<P, false, false, false, true>, dim3(grid), dim3(fmha_threads<false, true>()), kFmhaSmem, stream, tq, tk, tv, tk2, tv2, to, p); break;
-    LN3_FMHA_CASE2(0) LN3_FMHA_CASE2(2) LN3_FMHA_CASE2(3) LN3_FMHA_CASE2(4)
-#undef LN3_FMHA_CASE2
-    default: return set_error(LN3_EINVAL, "fmha: bad variant");
-  }
-  cudaError_t e = le != cudaSuccess ? le : cudaGetLastError();
+  cudaError_t e = launch_pdl(fmha_fwd_kernel, dim3(grid), dim3(kThreads), kSmem, stream, tq, tk, tv, tk2, tv2, to, p);
+  if (e == cudaSuccess) e = cudaGetLastError();
   if (e != cudaSuccess) return set_error(LN3_ECUDA, "fmha launch: %s", cudaGetErrorString(e));
   count_launch();
   return LN3_OK;

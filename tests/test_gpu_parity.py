@@ -92,9 +92,15 @@ def test_gemm_rejects_bad_shapes(dev):
 
 
 # ------------------------------------------------------------------ attention
+# (1,1,384,96) / (1,1,385,97): exactly one 384-row work item and one 96-row KV block, and one row / key past
+# them; (5,3,129,191): ragged everywhere; (16,16,768,768), (24,16,256,256), (8,16,768,768): the DiT self-attention
+# and decoder in-plane / global shapes -- on 148 SMs the first ends in a round of 68 items, which runs on the
+# (2 tiles | 1 tile) tail schedule, and the in-plane shape has a ragged last KV block and an empty third tile
 @pytest.mark.parametrize("B,H,Lq,Lkv", [(2, 12, 768, 768), (2, 16, 768, 77), (1, 4, 200, 333),
                                         (2, 16, 768, 1024), (3, 16, 256, 256), (1, 2, 1, 1),
-                                        (13, 16, 768, 768), (16, 16, 700, 77), (9, 16, 300, 130)])
+                                        (13, 16, 768, 768), (16, 16, 700, 77), (9, 16, 300, 130),
+                                        (1, 1, 384, 96), (1, 1, 385, 97), (5, 3, 129, 191),
+                                        (16, 16, 768, 768), (24, 16, 256, 256), (8, 16, 768, 768)])
 def test_fmha(dev, B, H, Lq, Lkv):
     from ln3diff_b200 import ops
     g = torch.Generator().manual_seed(Lq * 7 + Lkv)
@@ -106,6 +112,38 @@ def test_fmha(dev, B, H, Lq, Lkv):
     qf, kf, vf = (t.float().reshape(B, -1, H, 64).transpose(1, 2) for t in (q, k, v))
     ref = F.scaled_dot_product_attention(qf, kf, vf).transpose(1, 2).reshape(B, Lq, D)
     assert _rel(out, ref) < 6e-3
+
+
+def test_fmha_peaked_scores(dev):
+    """Inputs 3x the unit scale make later KV blocks exceed the running row maximum by more than the lazy-rescale
+    threshold (2^8), so blocks are redone against the new maximum and O is rescaled in tensor memory."""
+    from ln3diff_b200 import ops
+    g = torch.Generator().manual_seed(5)
+    B, H, L = 2, 4, 768
+    D = H * 64
+    qkv = (torch.randn(B, L, 3 * D, generator=g) * 3.0).bfloat16()
+    dq = qkv.to(dev)
+    out = ops.fmha(dq[:, :, :D], dq[:, :, D:2 * D], dq[:, :, 2 * D:], H)
+    qf, kf, vf = (t.float().reshape(B, -1, H, 64).transpose(1, 2) for t in (qkv[:, :, :D], qkv[:, :, D:2 * D],
+                                                                            qkv[:, :, 2 * D:]))
+    ref = F.scaled_dot_product_attention(qf, kf, vf).transpose(1, 2).reshape(B, L, D)
+    assert _rel(out, ref) < 8e-3
+
+
+# second K/V source appended after the first: a ragged first source (its last block is masked like a final
+# one) and the I23D shape (768 latent + 256 DINO tokens)
+@pytest.mark.parametrize("B,H,Lq,L1,L2", [(2, 4, 200, 256, 77), (1, 2, 100, 100, 50), (2, 16, 768, 768, 256)])
+def test_fmha_second_kv(dev, B, H, Lq, L1, L2):
+    from ln3diff_b200 import ops
+    g = torch.Generator().manual_seed(17 + L1)
+    D = H * 64
+    q = torch.randn(B, Lq, D, generator=g).bfloat16()
+    k1, v1 = torch.randn(B, L1, D, generator=g).bfloat16(), torch.randn(B, L1, D, generator=g).bfloat16()
+    k2, v2 = torch.randn(B, L2, D, generator=g).bfloat16(), torch.randn(B, L2, D, generator=g).bfloat16()
+    out = ops.fmha(q.to(dev), k1.to(dev), v1.to(dev), H, k2=k2.to(dev), v2=v2.to(dev))
+    sp = lambda t_: t_.float().reshape(B, -1, H, 64).transpose(1, 2)
+    ref = F.scaled_dot_product_attention(sp(q), sp(torch.cat([k1, k2], 1)), sp(torch.cat([v1, v2], 1)))
+    assert _rel(out, ref.transpose(1, 2).reshape(B, Lq, D)) < 6e-3
 
 
 # ------------------------------------------------------------------ elementwise
@@ -442,7 +480,7 @@ def test_latent_to_pixels_end_to_end(dev, golden):
 
 
 # ------------------------------------------------------------------ I23D (flow matching)
-def test_gemm_head_rmsnorm_and_fmha_second_kv(dev):
+def test_gemm_head_rmsnorm(dev):
     from ln3diff_b200 import ops
     from oracle import dit as odit
     g = torch.Generator().manual_seed(17)
@@ -456,14 +494,6 @@ def test_gemm_head_rmsnorm_and_fmha_second_kv(dev):
     ref[:, 1] = odit.rms_norm(ref[:, 1], nw[1], 1e-5)
     out = ops.gemm(a.to(dev), w.to(dev), b.to(dev), head_norm=nw.to(dev), head_norm_sec_cols=D)
     assert _rel(out, ref.reshape(M, 3 * D)) < 4e-3
-    B, Lq, L1, L2 = 2, 200, 256, 77
-    q = torch.randn(B, Lq, D, generator=g).bfloat16()
-    k1, v1 = torch.randn(B, L1, D, generator=g).bfloat16(), torch.randn(B, L1, D, generator=g).bfloat16()
-    k2, v2 = torch.randn(B, L2, D, generator=g).bfloat16(), torch.randn(B, L2, D, generator=g).bfloat16()
-    out = ops.fmha(q.to(dev), k1.to(dev), v1.to(dev), H, k2=k2.to(dev), v2=v2.to(dev))
-    sp = lambda t_: t_.float().reshape(B, -1, H, 64).transpose(1, 2)
-    ref = F.scaled_dot_product_attention(sp(q), sp(torch.cat([k1, k2], 1)), sp(torch.cat([v1, v2], 1)))
-    assert _rel(out, ref.transpose(1, 2).reshape(B, Lq, D)) < 6e-3
 
 
 def test_dit_i23d_forward_matches_reference_golden(dev, golden):

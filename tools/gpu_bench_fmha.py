@@ -1,4 +1,6 @@
-"""FMHA timings (self 768x768, cross 768x77) at the DiT-L/2 B'=16 shape; LN3_FMHA_POLY selects the variant."""
+"""FMHA timings at the shapes of the sampling paths: DiT-L/2 self-attention (16 samples) and cond-only
+cross-attention (8 samples, 77 text tokens), DiT2 decoder in-plane (24 x 256 tokens) and global (8 x 768)
+attention at 8 latents, and I23D self-attention over 768 latent + 256 DINO tokens (16 samples)."""
 import os
 import sys
 
@@ -9,11 +11,11 @@ from ln3diff_b200 import ops
 
 dev = "cuda"
 torch.manual_seed(0)
-B, H, L = 16, 16, 768
+H, D = 16, 16 * 64
 
 
-def timeit(fn, iters=20):
-    for _ in range(3):
+def timeit(fn, iters=30):
+    for _ in range(5):
         fn()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -25,15 +27,23 @@ def timeit(fn, iters=20):
     return e0.elapsed_time(e1) / iters * 1e3
 
 
-qkv = (torch.randn(B, L, 3 * H * 64, device=dev) * 0.5).bfloat16()
-q, k, v = qkv[:, :, :H * 64], qkv[:, :, H * 64:2 * H * 64], qkv[:, :, 2 * H * 64:]
-us = timeit(lambda: ops.fmha(q, k, v, H))
-out = ops.fmha(q, k, v, H)
-qf, kf, vf = (t.float().reshape(B, -1, H, 64).transpose(1, 2) for t in (q, k, v))
-ref = torch.nn.functional.scaled_dot_product_attention(qf, kf, vf).transpose(1, 2).reshape(B, L, H * 64)
-rel = ((out.float() - ref).norm() / ref.norm()).item()
-qc = (torch.randn(B, L, H * 64, device=dev) * 0.5).bfloat16()
-kvc = (torch.randn(B, 77, 2 * H * 64, device=dev) * 0.5).bfloat16()
-us2 = timeit(lambda: ops.fmha(qc, kvc[:, :, :H * 64], kvc[:, :, H * 64:], H))
-print(f"mma2={os.environ.get('LN3_FMHA_MMA2','1')} tail={os.environ.get('LN3_FMHA_TAIL','1')} ptmem={os.environ.get('LN3_FMHA_PTMEM','0')} split={os.environ.get('LN3_FMHA_SPLIT','0')} pp={os.environ.get('LN3_FMHA_PINGPONG','0')} poly={os.environ.get('LN3_FMHA_POLY', 'default')} self {us:.1f} us ({4.0 * B * H * L * L * 64 / us / 1e6:.0f} TF/s) "
-      f"rel {rel:.2e}; cross {us2:.1f} us", flush=True)
+def self_attn(B, L):
+    qkv = (torch.randn(B, L, 3 * D, device=dev) * 0.5).bfloat16()
+    return lambda: ops.fmha(qkv[:, :, :D], qkv[:, :, D:2 * D], qkv[:, :, 2 * D:], H)
+
+
+qc = (torch.randn(8, 768, D, device=dev) * 0.5).bfloat16()
+kvc = (torch.randn(8, 77, 2 * D, device=dev) * 0.5).bfloat16()
+qi = (torch.randn(16, 768, 3 * D, device=dev) * 0.5).bfloat16()
+kd = (torch.randn(16, 256, 2 * D, device=dev) * 0.5).bfloat16()
+cases = [
+    ("self(16x16x768x768)", 16 * 768 * 768, self_attn(16, 768)),
+    ("cross(8x16x768x77)", 8 * 768 * 77, lambda: ops.fmha(qc, kvc[:, :, :D], kvc[:, :, D:], H)),
+    ("inplane(24x16x256x256)", 24 * 256 * 256, self_attn(24, 256)),
+    ("global(8x16x768x768)", 8 * 768 * 768, self_attn(8, 768)),
+    ("i23d(16x16x768x(768+256))", 16 * 768 * 1024,
+     lambda: ops.fmha(qi[:, :, :D], qi[:, :, D:2 * D], qi[:, :, 2 * D:], H, k2=kd[:, :, :D], v2=kd[:, :, D:])),
+]
+for name, qk_pairs, fn in cases:
+    us = timeit(fn)
+    print(f"{name} {us:.1f} us ({4.0 * H * qk_pairs * 64 / us / 1e6:.0f} TF/s)", flush=True)

@@ -1,6 +1,6 @@
 // Timeline dump of the FMHA kernel (CTA 0): build with
-//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -DLN3_FMHA_TRACE -Iinclude -Iln3diff_b200/csrc \
-//        tools/microbench/fmha_trace.cu ln3diff_b200/csrc/*.cu -o tools/microbench/fmha_trace
+//   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 --expt-relaxed-constexpr -DLN3_FMHA_TRACE \
+//        -Iinclude -Iln3diff_b200/csrc tools/microbench/fmha_trace.cu ln3diff_b200/csrc/*.cu -o tools/microbench/fmha_trace
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
@@ -8,7 +8,7 @@
 #include <cuda_runtime.h>
 
 #include "ln3b200.h"
-namespace ln3 { int fmha_trace_copy(long long* host); int fmha3_trace_copy(long long* host); }
+namespace ln3 { int fmha_trace_copy(long long* host); }
 
 int main(int argc, char** argv) {
   const int B = 16, H = 16, L = 768, Lkv = argc > 1 ? atoi(argv[1]) : 768;
@@ -31,35 +31,20 @@ int main(int argc, char** argv) {
   for (int i = 0; i < 3; ++i)
     if (ln3_fmha_fwd(&a, nullptr) != 0) { printf("error: %s\n", ln3_last_error()); return 1; }
   cudaDeviceSynchronize();
-  const char* kv = getenv("LN3_FMHA_KERNEL");
-  if (kv && atoi(kv) == 2) {
-    static long long tr[3][64][12];
-    if (ln3::fmha_trace_copy(&tr[0][0][0])) { printf("trace copy failed\n"); return 1; }
-    long long t0 = tr[2][0][0];
-    printf("# role blk: slots (cycles since first event)\n");
-    for (int g = 0; g < 30; ++g) {
-      for (int r = 0; r < 3; ++r) {
-        printf("%s g=%2d:", r == 0 ? "WG0" : r == 1 ? "WG1" : "MMA", g);
-        for (int s = 0; s < (r == 2 ? 7 : 11); ++s) printf(" %7lld", tr[r][g][s] - t0);
-        printf("\n");
+  // WG slots 0 wait S | 1 S ready | 2 S in regs | 3 max done | 4 o_full(prev) | 6 exps done | 7 P handed |
+  // 8-10 epilogue (slot 5 is not recorded); MMA slots 0-2 QK_t issued | 3/5/7 p_full_t seen | 4/6/8 PV_t issued
+  static long long tr[4][64][12];
+  if (ln3::fmha_trace_copy(&tr[0][0][0])) { printf("trace copy failed\n"); return 1; }
+  long long t0 = tr[3][0][0];
+  printf("# role blk: slots (cycles since first event)\n");
+  for (int g = 0; g < 26; ++g) {
+    for (int r = 0; r < 4; ++r) {
+      printf("%s g=%2d:", r == 0 ? "WG0" : r == 1 ? "WG1" : r == 2 ? "WG2" : "MMA", g);
+      for (int s = 0; s < (r == 3 ? 9 : 11); ++s) {
+        const long long v = tr[r][g][s];
+        if (v == 0) printf("       -"); else printf(" %7lld", v - t0);
       }
-    }
-  } else {
-    // three-warpgroup kernel: WG slots 0 wait S | 1 S ready | 2 S in regs | 3 max done | 4 o_full(prev) | 5 permit |
-    // 6 exps done | 7 P handed | 8-10 epilogue; MMA slots 0-2 QK_t issued | 3/5/7 p_full_t seen | 4/6/8 PV_t issued
-    static long long tr[4][64][12];
-    if (ln3::fmha3_trace_copy(&tr[0][0][0])) { printf("trace copy failed\n"); return 1; }
-    long long t0 = tr[3][0][0];
-    printf("# role blk: slots (cycles since first event)\n");
-    for (int g = 0; g < 26; ++g) {
-      for (int r = 0; r < 4; ++r) {
-        printf("%s g=%2d:", r == 0 ? "WG0" : r == 1 ? "WG1" : r == 2 ? "WG2" : "MMA", g);
-        for (int s = 0; s < (r == 3 ? 9 : 11); ++s) {
-          const long long v = tr[r][g][s];
-          if (v == 0) printf("       -"); else printf(" %7lld", v - t0);
-        }
-        printf("\n");
-      }
+      printf("\n");
     }
   }
   return 0;
